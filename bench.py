@@ -377,6 +377,28 @@ def cfg5_leg(torch, dist, dev, rank, world, local_rank, reps=5):
         c5.close()
 
 
+DUMP_BYTES = 64 << 20
+SUMMARY_FIELDS = ("initial_cost", "final_cost", "iterations", "num_successful_steps", "termination", "imu_redo_count",
+                  "final_radius")
+
+
+def dump_outputs(out_dir, ctx, summaries, budget=DUMP_BYTES, suffix=""):
+    """What the last timed step handed its caller: the estimates of every window (poses, speed/bias, landmarks, landmark
+    quality) and the solver summaries (solve_time_s left out: it is a host timing), one float64 .npy per array.  When
+    all windows exceed `budget` bytes, a fixed seeded sample of windows is written; window_index.npy says which."""
+    n = len(summaries)
+    per_window = sum(v.nbytes for v in ctx.download(0).values()) + 8 * (len(SUMMARY_FIELDS) + 1)
+    keep = n if n * per_window <= budget else max(1, budget // per_window)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).permutation(n)[:keep])
+    states = [ctx.download(int(i)) for i in idx]
+    arrays = {k: np.stack([s[k] for s in states]) for k in ("poses", "speed_bias", "landmarks", "quality")}
+    arrays.update({k: np.array([summaries[i][k] for i in idx], np.float64) for k in SUMMARY_FIELDS})
+    arrays["window_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + suffix + ".npy"), v.astype(np.float64))
+
+
 def run_b200(args):
     import torch
     from okvis_b200 import capi
@@ -423,7 +445,8 @@ def run_b200(args):
     with torch.cuda.stream(stream):
         ev0.record(stream)
         for _ in range(args.steps):
-            iters += sum(s["iterations"] for s in step())
+            last = step()
+            iters += sum(s["iterations"] for s in last)
         ev1.record(stream)
     barrier()
     elapsed_ms = ev0.elapsed_time(ev1)
@@ -431,6 +454,8 @@ def run_b200(args):
     ctx.profile_enable(False)
     launches = ctx.kernel_launches - launches0
     clocks = sampler.result() if rank == 0 else None
+    if args.dump_outputs:       # before the e2e leg reuses these slots
+        dump_outputs(args.dump_outputs, ctx, last, DUMP_BYTES // world, "" if world == 1 else "_rank%d" % rank)
 
     # ---- e2e through the C-ABI with HOST buffers, resident windows (SURVEY 8f-3): the windows live on the device; every
     # step the host restores a slot to its uploaded estimates (okb_window_reset, device side), drops the newest frame
@@ -592,7 +617,14 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="tuning runs only: shrink the cpu_baseline sample to one window")
     ap.add_argument("--host-threads", type=int, default=12, help="host threads packing/uploading windows in the e2e leg")
     ap.add_argument("--distinct", type=int, default=8, help="distinct synthetic windows per rank (replicated to fill the batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the estimates and summaries of the last timed step to DIR/<name>.npy (float64, <= 64 MB "
+                         "in all) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computed")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,96 +1,78 @@
 """CPU: the oracle's restatement of DenseMatcher::match against the REAL reference matcher -- okvis_matcher's own sources
-compiled unmodified from /root/reference into oracle/_ref/libokvis_matcher_ref.so (oracle/Makefile.ref; the one part of the
-reference that builds with this image's toolchain).  Bit-exact match sets on tie-heavy random inputs, with skips, all
-numBest values, absolute and ratio thresholds, and through the Hamming distance.  Skipped where the reference tree is
-absent and no prebuilt library travelled (the GPU box)."""
-import ctypes as C
+compiled unmodified (oracle/Makefile.ref; the one part of the reference that builds without Eigen / Ceres / OpenCV).  What
+the reference answered is stored in tests/golden/matcher_reference_matrices.npz; the seeded inputs come from
+tools/make_golden_matcher.py, which wrote the answers, and are checked against the digests stored beside them.  Bit-exact
+match sets on tie-heavy random inputs, with skips, all numBest values, absolute and ratio thresholds, and through the
+Hamming distance."""
 import os
-import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SO = os.path.join(ROOT, "oracle", "_ref", "libokvis_matcher_ref.so")
+FIX = os.path.join(ROOT, "tests", "golden", "matcher_reference_matrices.npz")
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+import make_golden_matcher as G  # noqa: E402
 
 
 @pytest.fixture(scope="module")
 def ref():
-    if os.path.isdir("/root/reference/okvis_matcher"):
-        subprocess.run(["make", "-s", "-f", "Makefile.ref"], cwd=os.path.join(ROOT, "oracle"), check=True)
-    if not os.path.exists(SO):
-        pytest.skip("reference matcher library not built (no /root/reference here)")
-    lib = C.CDLL(SO)
-    lib.okr_match.restype = C.c_int
-
-    def match(D, skipA=None, skipB=None, threshold=4.0, num_best=4, use_ratio=False, ratio_threshold=3.0, threads=1):
-        D = np.ascontiguousarray(D, np.float32)
-        nA, nB = D.shape
-        a, d = np.zeros(nB, np.int32), np.zeros(nB, np.float32)
-        sa = np.ascontiguousarray(skipA, np.uint8) if skipA is not None else None
-        sb = np.ascontiguousarray(skipB, np.uint8) if skipB is not None else None
-        n = lib.okr_match(C.c_void_p(D.ctypes.data), nA, nB, C.c_void_p(sa.ctypes.data) if sa is not None else None,
-                          C.c_void_p(sb.ctypes.data) if sb is not None else None, C.c_float(threshold), num_best, int(use_ratio),
-                          C.c_float(ratio_threshold), threads, C.c_void_p(a.ctypes.data), C.c_void_p(d.ctypes.data))
-        return sorted((int(a[b]), b, float(d[b])) for b in range(nB) if a[b] >= 0), n
-    return match
+    return np.load(FIX)
 
 
 def oracle_set(o):
     return sorted((int(a), int(b), float(d)) for (a, b), d in zip(o["matches"], o["distances"]))
 
 
-def test_reference_known_answers_on_the_reference_itself(ref):
+def ref_set(m):
+    return [(int(a), int(b), float(d)) for a, b, d in m]
+
+
+def test_reference_known_answers_on_the_reference_itself(ref, oracle):
     """testMatcher.cpp:69-155 on the compiled reference: the fixture the oracle is pinned with really is what the
-    reference computes."""
-    def dist(va, vb):
-        return np.abs(np.subtract.outer(np.array(va, float), np.array(vb, float))).astype(np.float32)
-    got, _ = ref(dist([1, 3, 2, 0.9], [18, 2.1, 4, 1]), skipA=[1, 0, 0, 0], threshold=4.0)
-    assert {(a, b) for a, b, _ in got} == {(1, 2), (2, 1), (3, 3)}
-    got, _ = ref(dist([8, 1, 3, 2, 0.9], [18, 2.1, 4, 1, 7]), skipA=[1, 0, 0, 0, 0], threshold=4.0, use_ratio=True, ratio_threshold=3.0)
-    assert {(a, b) for a, b, _ in got} == {(1, 3), (3, 1)}
+    reference computes, and the oracle computes it too."""
+    for j, ((D, skipA, use_ratio), want) in enumerate(zip(G.known_answer_inputs(), ({(1, 2), (2, 1), (3, 3)}, {(1, 3), (3, 1)}))):
+        got = ref_set(ref["known%d_matches" % j])
+        assert {(a, b) for a, b, _ in got} == want
+        assert oracle_set(oracle.match_matrix(D, skipA, None, 4.0, 4, use_ratio, 3.0)) == got
 
 
 @pytest.mark.parametrize("num_best", [1, 2, 4, 8])
 @pytest.mark.parametrize("use_ratio", [False, True])
 def test_oracle_equals_reference_on_tie_heavy_matrices(ref, oracle, num_best, use_ratio):
-    rng = np.random.default_rng(100 + num_best + 10 * use_ratio)
-    for trial in range(60):
-        nA, nB = int(rng.integers(1, 60)), int(rng.integers(1, 60))
-        levels = int(rng.integers(2, 12))                                  # few distinct distances: ties everywhere
-        D = rng.integers(0, levels, (nA, nB)).astype(np.float32)
-        skipA = (rng.random(nA) < 0.1).astype(np.uint8)
-        skipB = (rng.random(nB) < 0.1).astype(np.uint8)
-        thr = float(rng.integers(1, levels + 1))
-        ratio = float(rng.choice([1.0, 1.5, 3.0]))
-        r, n = ref(D, skipA, skipB, thr, num_best, use_ratio, ratio)
+    k = "tie%d_%d_" % (num_best, use_ratio)
+    trials = G.tie_heavy_trials(num_best, use_ratio)
+    assert G.digest(*[a for t in trials for a in t[:3]], np.array([t[3:] for t in trials])) == str(ref[k + "inputs_sha256"]), \
+        "inputs differ from those the reference answered on"
+    counts, returned, m_all = ref[k + "counts"], ref[k + "returned"], ref[k + "matches"]
+    assert len(counts) == len(trials) == 60
+    off = 0
+    for trial, ((D, skipA, skipB, thr, ratio), cnt, n) in enumerate(zip(trials, counts, returned)):
+        r = ref_set(m_all[off:off + cnt])
+        off += cnt
         o = oracle.match_matrix(D, skipA, skipB, thr, num_best, use_ratio, ratio)
-        assert oracle_set(o) == r, (trial, nA, nB, thr)
+        assert oracle_set(o) == r, (trial, D.shape, thr)
         assert n == len(r)
+    assert off == len(m_all)
 
 
 def test_oracle_hamming_equals_reference_on_descriptor_distances(ref, oracle):
-    rng = np.random.default_rng(7)
-    for nA, nB, flips in ((300, 280, 30), (64, 512, 60), (500, 37, 12)):
-        base = rng.integers(0, 256, (max(nA, nB), 48), dtype=np.uint8)
-        A = base[:nA].copy()
-        B = base[rng.permutation(max(nA, nB))[:nB]].copy()
-        for row in B:
-            for i in rng.integers(0, 384, rng.integers(0, flips)):
-                row[i >> 3] ^= np.uint8(1 << (i & 7))
-        D = np.unpackbits(A[:, None, :] ^ B[None, :, :], axis=2).sum(2).astype(np.float32)
+    lists = G.hamming_lists()
+    assert G.digest(*[a for l in lists for a in l]) == str(ref["ham_inputs_sha256"]), "inputs differ from those the reference answered on"
+    for j, (A, B) in enumerate(lists):
         for use_ratio in (False, True):
-            r, _ = ref(D, None, None, 60.0, 4, use_ratio, 3.0)
+            r = ref_set(ref["ham%d_matches%d" % (j, use_ratio)])
             o = oracle.match_hamming(A, B, None, None, threshold=60.0, num_best=4, use_ratio=use_ratio, ratio_threshold=3.0)
             assert oracle_set(o) == r
 
 
-def test_four_reference_threads_agree_with_the_sequential_order_on_these_inputs(ref):
+def test_four_reference_threads_agree_with_the_sequential_order_on_these_inputs(ref, oracle):
     """The reference runs four matcher threads (Frontend.cpp:80) and its result can depend on their interleaving; the
     project's contract is the sequential order.  On inputs without contested ties the two coincide -- a sanity check that the
     threaded reference is the same algorithm, not a parity requirement."""
-    rng = np.random.default_rng(11)
-    D = rng.random((200, 180)).astype(np.float32) * 100.0                  # continuous distances: no ties
-    r1, _ = ref(D, threshold=30.0, threads=1)
-    r4, _ = ref(D, threshold=30.0, threads=4)
+    D = G.threads_matrix()
+    assert G.digest(D) == str(ref["threads_inputs_sha256"]), "inputs differ from those the reference answered on"
+    r1, r4 = ref_set(ref["threads_matches1"]), ref_set(ref["threads_matches4"])
     assert r1 == r4
+    assert oracle_set(oracle.match_matrix(D, threshold=30.0)) == r4
