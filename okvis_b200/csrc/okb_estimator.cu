@@ -442,7 +442,7 @@ static int upload_pack(okb_ctx* c, int win, const okb_window_desc* D) {
     }
     if (!(ob.sqrt_info > 0.0)) { c->set_error("observation with non-positive sqrt information"); return OKB_ERR_INVALID_ARG; }
   }
-  if (smemA2_bytes(K, 4 * ((6 * K + 1 + 3) / 4), 0) > (size_t)c->smem_optin) { c->set_error("window does not fit kernel A shared memory"); return OKB_ERR_CAPACITY; }
+  if (smemA2_bytes(K, 0) > (size_t)c->smem_optin) { c->set_error("window does not fit kernel A shared memory"); return OKB_ERR_CAPACITY; }
 
   WinStore& S = c->wins[win];
   S.uploaded = false;        // true again only when the whole upload has been issued successfully
@@ -567,7 +567,7 @@ extern "C" int okb_window_add_frame(okb_ctx* c, int win, const double* pose, con
   if (rc) return rc;
   const int K1 = W->K + 1, NSB1 = W->NSB + (speed_bias ? 1 : 0);
   if (K1 > S->caps.K || NSB1 > S->caps.K || 6 * K1 + 9 * NSB1 > kMaxDense) { c->set_error("okb_window_add_frame: frame capacity exceeded (okb_window_reserve)"); return OKB_ERR_CAPACITY; }
-  if (smemA2_bytes(K1, 4 * ((6 * K1 + 1 + 3) / 4), 0) > (size_t)c->smem_optin) { c->set_error("window does not fit kernel A shared memory"); return OKB_ERR_CAPACITY; }
+  if (smemA2_bytes(K1, 0) > (size_t)c->smem_optin) { c->set_error("window does not fit kernel A shared memory"); return OKB_ERR_CAPACITY; }
   if (term) {
     if ((int)term->pose0 >= K1 || (int)term->pose1 >= K1 || (int)term->sb0 >= NSB1 || (int)term->sb1 >= NSB1 ||
         (uint64_t)term->sample_offset + term->sample_count > (uint64_t)n_samples || term->sample_count < 2) {
@@ -1087,26 +1087,26 @@ extern "C" int okb_window_reset(okb_ctx* c, int first, int count) {
 // Launch geometry of one optimize of windows [first, first+count): everything a captured CUDA graph depends on
 // besides the kernel arguments.
 struct RoundPlan {
-  int max_chunks = 1, max_imu = 0, max_cx = 1, max_K = 1, acc_copies = 1, chol_smem = 1, solve_threads = S_THREADS, gxQ = 1, shard = 0, push_gx = 1;
+  int max_chunks = 1, max_imu = 0, max_cx = 1, max_K = 1, acc_smem = 1, chol_smem = 1, solve_threads = S_THREADS, gxQ = 1, shard = 0, push_gx = 1;
   size_t smA = 0, smS = 0, smQ = 0;
 };
 static int plan_rounds(okb_ctx* c, int first, int count, RoundPlan& P) {
   P = RoundPlan();
   int chol_smem = 1;       // solve_mode of k_solve: 1 system in shared memory, 2 pose system + chain band, 0 chain band only
   // Schur accumulator in shared memory if two CTAs per SM still fit (else one CTA; else accumulate in global memory)
-  int acc_copies = 1;
+  int acc_smem = 1;
   const size_t sm_two = ((size_t)c->smem_per_sm - 2048) / 2;
   for (int i = first; i < first + count; ++i)
-    if (smemA2_bytes(c->host[i].K, c->host[i].dcp, 1) > std::min((size_t)c->smem_optin, sm_two) &&
-        smemA2_bytes(c->host[i].K, c->host[i].dcp, 0) <= sm_two) acc_copies = 0;
+    if (smemA2_bytes(c->host[i].K, 1) > std::min((size_t)c->smem_optin, sm_two) &&
+        smemA2_bytes(c->host[i].K, 0) <= sm_two) acc_smem = 0;
   for (int i = first; i < first + count; ++i)
-    if (smemA2_bytes(c->host[i].K, c->host[i].dcp, acc_copies) > (size_t)c->smem_optin) acc_copies = 0;
+    if (smemA2_bytes(c->host[i].K, acc_smem) > (size_t)c->smem_optin) acc_smem = 0;
   int maxL = 1;
   for (int i = first; i < first + count; ++i) {
     const WinDev& W = c->host[i];
     P.max_chunks = std::max(P.max_chunks, W.n_chunks);
     P.max_imu = std::max(P.max_imu, W.n_imu);
-    P.smA = std::max(P.smA, smemA2_bytes(W.K, W.dcp, acc_copies));
+    P.smA = std::max(P.smA, smemA2_bytes(W.K, acc_smem));
     P.max_cx = std::max(P.max_cx, (W.L + L1_THREADS - 1) / L1_THREADS);
     P.max_K = std::max(P.max_K, W.K);
     {      // the roomiest mode this window fits; the range runs in the most modest one (1 > 2 > 0)
@@ -1135,7 +1135,7 @@ static int plan_rounds(okb_ctx* c, int first, int count, RoundPlan& P) {
       if (P.smS > (size_t)c->smem_optin) { c->set_error("window does not fit kernel S shared memory"); return OKB_ERR_CAPACITY; }
     }
   }
-  P.acc_copies = acc_copies; P.chol_smem = chol_smem;
+  P.acc_smem = acc_smem; P.chol_smem = chol_smem;
   P.solve_threads = (2 * count <= c->sm_count) ? 512 : S_THREADS;      // few windows: one wide CTA per SM (all ranks of a sharded window choose alike)
   P.gxQ = std::max(1, std::min((maxL + 127) / 128, (4 * c->sm_count + count - 1) / count));
   P.shard = c->shard_world > 1 ? 1 : 0;
@@ -1160,7 +1160,7 @@ static int launch_rounds(okb_ctx* c, int first, int count, const okb_solve_optio
     prof_begin(c, 0);
     k_linearize<<<dim3(P.max_cx, P.max_K, count), L1_THREADS, 0, c->stream>>>(c->d_wins, first);
     k_lmblock<<<dim3(P.max_cx, count), 128, 0, c->stream>>>(c->d_wins, first);
-    k_schur<<<gridA, A2_THREADS, P.smA, c->stream>>>(c->d_wins, first, P.acc_copies, opt.max_iterations);
+    k_schur<<<gridA, A2_THREADS, P.smA, c->stream>>>(c->d_wins, first, P.acc_smem, opt.max_iterations);
     if (P.shard) {    // chunk reduction fused with the push half of the all-reduce over peer memory
       k_shard_push<<<dim3(P.push_gx, count), 256, 0, c->stream>>>(c->d_wins, first);
       c->launches += 1;

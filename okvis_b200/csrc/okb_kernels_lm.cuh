@@ -6,8 +6,8 @@
 //       do not see the frame exit immediately (landmarks are sorted by observing-frame range).
 //   k_lmblock ("A1b"): one thread per landmark: H_ll = sum_f M_f, (H_ll + mu E)^-1 by 3x3 Cholesky.
 //   k_schur ("A2"): one CTA per (landmark chunk, window), tiles of 32 landmarks staged by TMA bulk copies:
-//       Y_f = W_f L^-T into a shared-memory tile, then the Schur complement as a block-sparse SYRK
-//       S += Y Y^T with one lane per 6x6 frame-block pair (details at the kernel).
+//       Y_f = W_f L^-T into a tile-local shared-memory tile, then the Schur complement as a SYRK S += Y Y^T
+//       over 8x8 blocks on the FP64 tensor cores (details at the kernel).
 //   k_quality: post-solve landmark quality (Estimator.cpp:880-894), one thread per landmark.
 #pragma once
 #include "okb_estimator.cuh"
@@ -15,7 +15,7 @@
 namespace okb {
 
 constexpr int L1_THREADS = 128;          // k_linearize block = landmarks per CTA (x one frame)
-constexpr int A2_THREADS = 192;          // k_schur block (6 warps at 168 registers: two CTAs per SM)
+constexpr int A2_THREADS = 256;          // k_schur block (8 warps, two CTAs per SM)
 constexpr int A2_TILE = 32;              // landmarks per Y tile
 constexpr int kPartH = 32;               // doubles per (cx, frame) record: 27 H_pp/g_p + cost + stepnorm2 + pad
 
@@ -267,31 +267,35 @@ __global__ void __launch_bounds__(128) k_lmblock(const WinDev* __restrict__ wins
 // reduced right-hand side).
 //
 // Landmarks arrive sorted by (first, last) observing frame, so a tile of 32 consecutive landmarks only
-// touches the frames [a, b] listed in W.tile_range.  The SYRK is done per 6x6 frame block: one lane owns one
-// block pair (36 accumulators in registers, 12 operand doubles per 36 multiply-adds) and KS <= 8 adjacent
-// lanes of the same warp split the tile's 96 columns.  The lane -> block-pair map covers the frames
-// [a, K-1] and is rebuilt only when the tile's first frame a changes (landmarks are sorted by it: at most K
-// times per chunk); lanes whose pair reaches beyond the tile's last frame b sit the tile out, and since pairs
-// are dealt to the warps row-major, whole warps skip narrow tiles.  On a rebuild the accumulators are summed
-// over the KS lanes with shuffles (fixed order) and added by one lane to the chunk's packed accumulator in
-// shared memory (or to the global partial for windows with many frames): one writer per element, no barrier
-// => deterministic.
+// touches the frames [fa, fb] listed in W.tile_range.  Y is built tile-local in shared memory, k-major (column
+// k = 3 * landmark + c): local row 6(f - fa) + i is pose row 6f + i, local row 6u (u = fb - fa + 1) is the
+// augmented row, and rows up to the next multiple of 8 are zero (see schur_ldy).  The SYRK runs on the FP64 tensor cores
+// (mma.sync.m8n8k4.f64) over the T = ceil((6u+1)/8) block rows: the lower-triangle 8x8 blocks are dealt to the
+// warps as contiguous row-major ranges (at most one block above the average; neighbours share a block row, so
+// the A fragment is loaded once for both), two blocks interleaved per warp.  The owning lane adds its fragment
+// to the chunk's packed accumulator in shared memory (or to the global partial for windows with many frames):
+// the local -> global row map is monotone and injective, so there is one writer per element per tile, and
+// tiles are separated by the tile loop's barriers => deterministic.
 // ------------------------------------------------------------------------------------------------
 constexpr int kLiStride = 9;   // L^-1 (6) | z (3), as in global memory (one bulk copy per tile)
 
-__host__ __device__ inline int schur_ldy(int dcp) { return dcp + 2; }   // Y row stride: rows shift by 16 B across banks
+// Y row stride (doubles): at least the 6K+1 rows of the widest tile, and 4 (mod 8) so that the DMMA fragment loads
+// (lane 4g + t reads t * ldy + g) and the Y-build double2 stores (4 landmarks x 2 frames per quarter warp) hit
+// distinct banks.  The padding rows of a full-width tile's last block row may reach beyond the stride: they alias the
+// first rows of the next column (or the 8-double pad after the tile) and only feed output entries that are dropped.
+__host__ __device__ inline int schur_ldy(int K) { return 6 * K + 1 + ((3 - 6 * K) & 7); }
 
-// acc_copies: 1 = the chunk's Schur accumulator (packed lower triangle of the (dc+1) x (dc+1) matrix) lives in
+// acc_smem: 1 = the chunk's Schur accumulator (packed lower triangle of the (dc+1) x (dc+1) matrix) lives in
 // shared memory; 0 = accumulate in the chunk's global partial instead (windows with many frames).
 __host__ __device__ inline size_t schur_acc_doubles(int K) { return (size_t)(6 * K + 1) * (6 * K + 2) / 2; }
-__host__ __device__ inline size_t smemA2_bytes(int K, int dcp, int acc_copies) {
+__host__ __device__ inline size_t smemA2_bytes(int K, int acc_smem) {
   size_t b = 16;                                                    // two mbarriers (TMA completion per buffer)
-  b += ((size_t)3 * A2_TILE * schur_ldy(dcp) + 8) * sizeof(double);   // Y tile, k-major (+ pad: the augmented-row lanes read 6 wide)
+  b += ((size_t)3 * A2_TILE * schur_ldy(K) + 8) * sizeof(double);  // Y tile, k-major (+ pad: the last block row of a full-width tile)
   b += (size_t)2 * K * 6 * A2_TILE * sizeof(double);               // M tiles [f][e][ll] (double buffered)
   b += (size_t)2 * A2_TILE * kLiStride * sizeof(double);           // L^-1 | z
   b += (size_t)2 * A2_TILE * 4 * sizeof(double);                   // X
   b += (size_t)K * 4 * sizeof(double);                             // frame translations
-  b += (size_t)acc_copies * schur_acc_doubles(K) * sizeof(double);
+  b += (size_t)acc_smem * schur_acc_doubles(K) * sizeof(double);
   return b;
 }
 
@@ -319,7 +323,12 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-__global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restrict__ wins, int win_first, int acc_copies, int max_iterations) {
+// C += A B on the FP64 tensor cores, fragment layout of m8n8k4 f64: lane 4g + t holds A[g][t], B[t][g], C[g][2t..2t+1]
+__device__ __forceinline__ void dmma_8x8x4(double& c0, double& c1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
+}
+
+__global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restrict__ wins, int win_first, int acc_smem, int max_iterations) {
   const WinDev& W = wins[win_first + blockIdx.y];
   SolverState* st = W.st;
   if (st->done) return;
@@ -330,7 +339,7 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
   if (chunk >= W.n_chunks) return;
   const int tid = threadIdx.x;
   const int K = W.K, dc = W.dc, dcp = W.dcp, L = W.L;
-  const int ldy = schur_ldy(dcp);
+  const int ldy = schur_ldy(K);
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
   uint64_t* mbar = reinterpret_cast<uint64_t*>(smem_raw);            // [2]: TMA completion of tile buffer 0 / 1
@@ -340,20 +349,19 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
   double* sXb = sLib + 2 * A2_TILE * kLiStride;
   double* tws = sXb + 2 * A2_TILE * 4;
   double* Sp = W.partA + (size_t)chunk * W.partA_stride;
-  const bool acc_smem = acc_copies > 0;
-  const int acc_n = (dc + 1) * (dc + 2) / 2;
-  double* Sacc = acc_smem ? tws + 4 * K : Sp;     // packed lower triangles in shared memory, or the global partial itself
-  const int n_acc = acc_smem ? acc_copies * acc_n : dcp * dcp;
+  double* Sacc = acc_smem ? tws + 4 * K : Sp;     // packed lower triangle in shared memory, or the global partial itself
+  const int n_acc = acc_smem ? (dc + 1) * (dc + 2) / 2 : dcp * dcp;
 
   for (int f = tid; f < K; f += A2_THREADS) {
     tws[4 * f] = W.pose_c[7 * f]; tws[4 * f + 1] = W.pose_c[7 * f + 1]; tws[4 * f + 2] = W.pose_c[7 * f + 2];
   }
   for (int i = tid; i < n_acc; i += A2_THREADS) Sacc[i] = 0.0;
+  if (tid < 8) Yt[(size_t)3 * A2_TILE * ldy + tid] = 0.0;
 
   const int lm_begin = chunk * W.lm_per_chunk;     // multiple of A2_TILE
   const int lm_end = min(L, lm_begin + W.lm_per_chunk);
 
-  // Asynchronous staging of one tile by the TMA engine (cp.async.bulk, issued by warp 0, completion on
+  // Asynchronous staging of one tile by the TMA engine (cp.async.bulk, issued by the last warp, completion on
   // mbar[buf]); frames [fa, fb] only.  Global and shared layouts agree, so every piece is one contiguous copy:
   //   M  [tile][f][6][32] -> sM[f][6][32] : frames [fa, fb] are one contiguous block
   //   Li [l][9] -> sLi[32][9] (2304 B),  X = lm_c [l][4] -> sX[32][4] (1024 B)
@@ -364,7 +372,7 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
   uint32_t phase_bits = 0;      // bit b: parity to wait for on mbar[b]
   auto stage = [&](int base, int buf, uint32_t tr) {
     const int fa = tr & 0xffu, fb = tr >> 8;
-    if (fa > fb || warp != A2_THREADS / 32 - 1) return;      // the last warp issues the copies (the first one also builds the augmented row)
+    if (fa > fb || warp != A2_THREADS / 32 - 1) return;      // the last warp issues the copies
     double* sM = sMb + (size_t)buf * K * 6 * A2_TILE;
     double* sLi = sLib + buf * A2_TILE * kLiStride;
     double* sX = sXb + buf * A2_TILE * 4;
@@ -378,85 +386,22 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
     }
   };
 
-  // ---- lane -> (block pair, column split) map of the current frame range: tid = kg * n_act + item
-  int cur_fa = -1, cur_fb = -1, lane_fmax = 0;
-  int KS = 1, kg = 0, n_act = 0, n_pairs = 0, n_pass = 1;
-  int a_off = 0, b_off = 0, row0 = 0, col0 = 0;
-  bool on = false, aug = false;
-  double acc[36];
-#pragma unroll
-  for (int i = 0; i < 36; ++i) acc[i] = 0.0;
-
-  auto decode = [&](int item, int fa) {
-    aug = false;
-    on = item < n_act;
-    if (!on) return;
-    if (item < n_pairs) {
-      int i = (int)((sqrtf(8.0f * (float)item + 1.0f) - 1.0f) * 0.5f);
-      while (i * (i + 1) / 2 > item) --i;
-      while ((i + 1) * (i + 2) / 2 <= item) ++i;
-      const int j = item - i * (i + 1) / 2;
-      row0 = 6 * (fa + i); col0 = 6 * (fa + j);
-      lane_fmax = fa + i;
-    } else {
-      aug = true;
-      row0 = dc; col0 = 6 * (fa + item - n_pairs);
-      lane_fmax = fa + item - n_pairs;
-    }
-    a_off = row0; b_off = col0;
-  };
-  // Adds the accumulators to the chunk accumulator and clears them.  Called at CTA-uniform points only.
-  // Shared-memory mode: column split kg owns copy kg, so all lanes add concurrently (a later flush that
-  // touches the same element from another lane is separated by the tile loop's barriers); the copies are
-  // summed in fixed order at the end => deterministic.  Global mode: KS rounds separated by barriers.
-  // Few instructions per element: flushes run on all 12 warps at once and are issue-bound.
-  double* Ssm = tws + 4 * K;
-  auto flush_smem = [&](int copy) {
-    double* cp = Ssm + (size_t)copy * acc_n + col0;
-    if (aug) {
-      double* rp = cp + (size_t)dc * (dc + 1) / 2;
-#pragma unroll
-      for (int c = 0; c < 6; ++c) rp[c] += acc[c];
-    } else if (row0 == col0) {        // diagonal block: lower triangle only
-#pragma unroll
-      for (int r = 0; r < 6; ++r) {
-        double* rp = cp + (size_t)(row0 + r) * (row0 + r + 1) / 2;
-#pragma unroll
-        for (int c = 0; c <= r; ++c) rp[c] += acc[r * 6 + c];
-      }
-    } else {
-#pragma unroll
-      for (int r = 0; r < 6; ++r) {
-        double* rp = cp + (size_t)(row0 + r) * (row0 + r + 1) / 2;
-        double t[6];
-#pragma unroll
-        for (int c = 0; c < 6; ++c) t[c] = rp[c];
-#pragma unroll
-        for (int c = 0; c < 6; ++c) rp[c] = t[c] + acc[r * 6 + c];
-      }
-    }
-  };
-  auto flush_global = [&]() {
-#pragma unroll
-    for (int i = 0; i < 36; ++i) {
-      const int rr = row0 + i / 6, cc = col0 + i % 6;
-      if ((!aug || i < 6) && cc <= rr) Sp[(size_t)rr * dcp + cc] += acc[i];
-    }
-  };
-  // The KS column splits of a block pair are adjacent lanes of one warp: they are summed with shuffles (fixed
-  // order) and the kg == 0 lane adds the result to the accumulator -- no barrier, one writer per element.
-  auto flush = [&]() {
-    // KS is a power of two: pairwise tree over the column splits (fixed shape => deterministic)
-    for (int o = KS >> 1; o > 0; o >>= 1) {
-#pragma unroll
-      for (int i = 0; i < 36; ++i) acc[i] += __shfl_down_sync(0xffffffffu, acc[i], o);
-    }
-    if (on && kg == 0) { if (acc_smem) flush_smem(0); else flush_global(); }
-#pragma unroll
-    for (int i = 0; i < 36; ++i) acc[i] = 0.0;
+  // Adds the fragment (c0, c1) of local block (bi, bj) to the chunk accumulator: lane 4g + t holds local row
+  // 8 bi + g, columns 8 bj + 2t and 8 bj + 2t + 1.  Padding rows, entries above the diagonal and the z z^T corner
+  // (not part of S) are dropped.
+  const int g = lane >> 2, t4 = lane & 3;
+  auto accumulate = [&](int bi, int bj, double c0, double c1, int row0, int nrow) {
+    const int i = 8 * bi + g;
+    if (i > nrow) return;
+    const int gr = i < nrow ? row0 + i : dc;
+    double* rp = Sacc + (acc_smem ? (size_t)gr * (gr + 1) / 2 : (size_t)gr * dcp) + row0;
+    const int j = 8 * bj + 2 * t4;
+    if (j <= i && j < nrow) rp[j] += c0;
+    if (j + 1 <= i && j + 1 < nrow) rp[j + 1] += c1;
   };
 
-#ifdef OKB_SCHUR_PROF     // per-phase cycle counters of chunk 0 / thread 0 (costs ~18 registers: diagnostics builds only)
+#ifdef OKB_SCHUR_PROF     // per-phase cycle counters of chunk 0 / thread 0 (diagnostics builds only): phase_ns[8 + i] for
+                          // i = 0 TMA wait + barrier, 1 copy issue, 2 Y build, 3 DMMA, 4 accumulate, 5 copy-out
   const bool prof = (tid == 0 && chunk == 0);
   unsigned long long t_ph = 0, ph[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   auto now = []() { return (unsigned long long)clock64(); };
@@ -484,55 +429,29 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
     __syncthreads();                       // the previous SYRK has finished (Y tile and the other buffer are free)
     SCHUR_MARK(0);
     if (base + A2_TILE < lm_end) stage(base + A2_TILE, buf ^ 1, tr_n1);   // overlaps with this tile's math
-    SCHUR_MARK(6);
+    SCHUR_MARK(1);
     const uint32_t tr = tr_cur;
     tr_cur = tr_n1; tr_n1 = tr_n2;
     const int fa = tr & 0xffu, fb = tr >> 8;
     buf ^= 1;
     if (fa > fb) continue;                 // no observed landmark in this tile (CTA-uniform)
-    const int u = fb - fa + 1;
-    // The lane -> block-pair map covers exactly the tile's frame range [fa, fb] and is rebuilt (after a flush of the
-    // register accumulators: a shuffle tree over the column splits + one shared-memory add per element) whenever the
-    // range changes.  Landmarks are sorted by (first, last) frame, so neighbouring tiles mostly share or shrink the
-    // range; every lane that is mapped does useful multiply-adds (narrow tiles get up to 8 column splits per pair).
-    if (fa != cur_fa || fb != cur_fb) {
-      flush();
-      cur_fa = fa; cur_fb = fb;
-      const int um = fb - fa + 1;
-      n_pairs = um * (um + 1) / 2;
-      n_act = n_pairs + um;
-      // block pairs are dealt to the warps (ipw per warp); inside a warp lane = pair * KS + split
-      constexpr int NW = A2_THREADS / 32;
-      const int ipw = (n_act + NW - 1) / NW;
-      if (ipw <= 32) {
-        n_pass = 1;
-        KS = 1;
-        while (2 * KS <= 8 && 2 * KS * ipw <= 32) KS *= 2;          // largest power of two that fits the warp
-        kg = lane % KS;
-        const int il = lane / KS;
-        decode(warp * ipw + il, fa);
-        on = on && il < ipw;
-      } else {                     // more block pairs than lanes (beyond 17 frames): one pair per lane, several passes
-        n_pass = (n_act + A2_THREADS - 1) / A2_THREADS;
-        KS = 1; kg = 0;
-      }
+    const int u = fb - fa + 1, nrow = 6 * u, row0 = 6 * fa;
+    const int T = (nrow + 8) >> 3;         // 8-row blocks covering the pose rows and z
+    // ---- augmented row z (local row nrow) and zero rows up to 8T (or the stride)
+    for (int i = tid; i < 3 * A2_TILE * (min(8 * T, ldy) - nrow); i += A2_THREADS) {
+      const int k = i % (3 * A2_TILE), r = nrow + i / (3 * A2_TILE), ll = k / 3;
+      Yt[(size_t)k * ldy + r] = (r == nrow && ll < nl) ? sLi[ll * kLiStride + 6 + k % 3] : 0.0;
     }
-    SCHUR_MARK(1);
-    // ---- augmented row z
-    if (tid < A2_TILE) {
-      const int ll = tid;
-      double* yz = Yt + (size_t)(3 * ll) * ldy + dc;
-      const bool v = ll < nl;
-      yz[0] = v ? sLi[ll * kLiStride + 6] : 0.0;
-      yz[ldy] = v ? sLi[ll * kLiStride + 7] : 0.0;
-      yz[2 * ldy] = v ? sLi[ll * kLiStride + 8] : 0.0;
-    }
-    // ---- Y_f = W_f L^-T for every (landmark, frame) pair of the tile, frames [fa, fb]
-    for (int pidx = tid; pidx < A2_TILE * u; pidx += A2_THREADS) {
-      const int ll = pidx % A2_TILE, f = fa + pidx / A2_TILE;      // landmark fastest: conflict-free reads of sM
-      double* y0 = Yt + (size_t)(3 * ll) * ldy + 6 * f;
-      double* y1 = y0 + ldy;
-      double* y2 = y1 + ldy;
+    // ---- Y_f = W_f L^-T for every (landmark, frame) pair of the tile, frames [fa, fb].  Pair p: bits 0-1 and 3-5
+    // are the landmark, bit 2 and bits 6.. the frame, so a quarter warp stores 4 landmarks x 2 frames
+    // (conflict-free double2 stores with ldy = 4 mod 8).
+    for (int p = tid; p < A2_TILE * ((u + 1) & ~1); p += A2_THREADS) {
+      const int ll = (p & 3) | ((p >> 1) & 28), fl = ((p >> 2) & 1) | ((p >> 5) & ~1);
+      if (fl >= u) continue;
+      const int f = fa + fl;
+      double2* y0 = reinterpret_cast<double2*>(Yt + (size_t)(3 * ll) * ldy + 6 * fl);
+      double2* y1 = reinterpret_cast<double2*>(Yt + (size_t)(3 * ll + 1) * ldy + 6 * fl);
+      double2* y2 = reinterpret_cast<double2*>(Yt + (size_t)(3 * ll + 2) * ldy + 6 * fl);
       double M0 = 0, M1 = 0, M2 = 0, M3 = 0, M4 = 0, M5 = 0;
       if (ll < nl) {
         const double* sp = sM + (size_t)(f * 6) * A2_TILE + ll;
@@ -545,61 +464,75 @@ __global__ void __launch_bounds__(A2_THREADS, 2) k_schur(const WinDev* __restric
         const double N00 = M0 * Li[0], N01 = M0 * Li[1] + M1 * Li[2], N02 = M0 * Li[3] + M1 * Li[4] + M2 * Li[5];
         const double N10 = M1 * Li[0], N11 = M1 * Li[1] + M3 * Li[2], N12 = M1 * Li[3] + M3 * Li[4] + M4 * Li[5];
         const double N20 = M2 * Li[0], N21 = M2 * Li[1] + M4 * Li[2], N22 = M2 * Li[3] + M4 * Li[4] + M5 * Li[5];
-        y0[0] = -w * N00; y0[1] = -w * N10; y0[2] = -w * N20;
-        y1[0] = -w * N01; y1[1] = -w * N11; y1[2] = -w * N21;
-        y2[0] = -w * N02; y2[1] = -w * N12; y2[2] = -w * N22;
-        y0[3] = -(p1 * N20 - p2 * N10); y0[4] = -(p2 * N00 - p0 * N20); y0[5] = -(p0 * N10 - p1 * N00);
-        y1[3] = -(p1 * N21 - p2 * N11); y1[4] = -(p2 * N01 - p0 * N21); y1[5] = -(p0 * N11 - p1 * N01);
-        y2[3] = -(p1 * N22 - p2 * N12); y2[4] = -(p2 * N02 - p0 * N22); y2[5] = -(p0 * N12 - p1 * N02);
+        y0[0] = make_double2(-w * N00, -w * N10); y0[1] = make_double2(-w * N20, -(p1 * N20 - p2 * N10));
+        y0[2] = make_double2(-(p2 * N00 - p0 * N20), -(p0 * N10 - p1 * N00));
+        y1[0] = make_double2(-w * N01, -w * N11); y1[1] = make_double2(-w * N21, -(p1 * N21 - p2 * N11));
+        y1[2] = make_double2(-(p2 * N01 - p0 * N21), -(p0 * N11 - p1 * N01));
+        y2[0] = make_double2(-w * N02, -w * N12); y2[1] = make_double2(-w * N22, -(p1 * N22 - p2 * N12));
+        y2[2] = make_double2(-(p2 * N02 - p0 * N22), -(p0 * N12 - p1 * N02));
       } else {
+        const double2 z = make_double2(0.0, 0.0);
 #pragma unroll
-        for (int i = 0; i < 6; ++i) { y0[i] = 0.0; y1[i] = 0.0; y2[i] = 0.0; }
+        for (int i = 0; i < 3; ++i) { y0[i] = z; y1[i] = z; y2[i] = z; }
       }
     }
-    SCHUR_MARK(2);
     __syncthreads();
-    SCHUR_MARK(3);
-    // ---- SYRK over the tile's 3*nl columns
-    const int ncols = 3 * nl;
-    for (int pass = 0; pass < n_pass; ++pass) {
-      if (n_pass > 1) decode(pass * A2_THREADS + tid, fa);
-      if (on && lane_fmax <= fb) {
-        const double* pa = Yt + a_off + (size_t)kg * ldy;
-        const double* pb = Yt + b_off + (size_t)kg * ldy;
-        const int step = KS * ldy;
-#pragma unroll 1
-        for (int k = kg; k < ncols; k += KS) {
-          const double2 a01 = *reinterpret_cast<const double2*>(pa);
-          const double2 a23 = *reinterpret_cast<const double2*>(pa + 2);
-          const double2 a45 = *reinterpret_cast<const double2*>(pa + 4);
-          const double2 b01 = *reinterpret_cast<const double2*>(pb);
-          const double2 b23 = *reinterpret_cast<const double2*>(pb + 2);
-          const double2 b45 = *reinterpret_cast<const double2*>(pb + 4);
-          const double av[6] = {a01.x, a01.y, a23.x, a23.y, a45.x, a45.y};
-          const double bv[6] = {b01.x, b01.y, b23.x, b23.y, b45.x, b45.y};
-#pragma unroll
-          for (int i = 0; i < 6; ++i)
-#pragma unroll
-            for (int j = 0; j < 6; ++j) acc[i * 6 + j] += av[i] * bv[j];
-          pa += step; pb += step;
+    SCHUR_MARK(2);
+    // ---- SYRK: this warp's range of the T(T+1)/2 lower-triangle blocks (row-major), two at a time, each over
+    // ceil(3 nl / 4) k-steps (columns from 3 nl on are zero)
+    const int ns = (3 * nl + 3) >> 2;
+    const int nb = T * (T + 1) / 2;
+    constexpr int NW = A2_THREADS / 32;
+    const int b_lo = warp * nb / NW, b_hi = (warp + 1) * nb / NW;
+    int bi = (int)((sqrtf(8.0f * (float)b_lo + 1.0f) - 1.0f) * 0.5f);
+    while (bi * (bi + 1) / 2 > b_lo) --bi;
+    while ((bi + 1) * (bi + 2) / 2 <= b_lo) ++bi;
+    int bj = b_lo - bi * (bi + 1) / 2;
+    const double* yl = Yt + (size_t)t4 * ldy + g;
+    const int kstep = 4 * ldy;
+    for (int b = b_lo; b < b_hi; b += 2) {
+      int bi1 = bi, bj1 = bj + 1;
+      if (bj1 > bi1) { ++bi1; bj1 = 0; }
+      double c00 = 0.0, c01 = 0.0, c10 = 0.0, c11 = 0.0;
+      const double* pa0 = yl + 8 * bi;
+      const double* pb0 = yl + 8 * bj;
+      const bool diag0 = bi == bj;
+      if (b + 1 < b_hi) {
+        const double* pa1 = yl + 8 * bi1;
+        const double* pb1 = yl + 8 * bj1;
+        const bool diag1 = bi1 == bj1, same_row = bi1 == bi;
+#pragma unroll 4
+        for (int s = 0; s < ns; ++s) {
+          const int o = s * kstep;
+          const double a0 = pa0[o];
+          const double b0 = diag0 ? a0 : pb0[o];
+          const double a1 = same_row ? a0 : pa1[o];
+          const double b1 = diag1 ? a1 : pb1[o];
+          dmma_8x8x4(c00, c01, a0, b0);
+          dmma_8x8x4(c10, c11, a1, b1);
+        }
+      } else {
+#pragma unroll 4
+        for (int s = 0; s < ns; ++s) {
+          const int o = s * kstep;
+          const double a0 = pa0[o];
+          const double b0 = diag0 ? a0 : pb0[o];
+          dmma_8x8x4(c00, c01, a0, b0);
         }
       }
-      if (n_pass > 1) flush();
+      SCHUR_MARK(3);
+      accumulate(bi, bj, c00, c01, row0, nrow);
+      if (b + 1 < b_hi) accumulate(bi1, bj1, c10, c11, row0, nrow);
+      SCHUR_MARK(4);
+      bi = bi1; bj = bj1 + 1;
+      if (bj > bi) { ++bi; bj = 0; }
     }
-    SCHUR_MARK(4);
   }
-  __syncthreads();
-  if (n_pass == 1) flush();
   if (acc_smem) {
     __syncthreads();
     for (int i = tid; i < (dc + 1) * dcp; i += A2_THREADS) {
       const int r = i / dcp, cidx = i % dcp;
-      if (cidx <= r) {
-        const int e = r * (r + 1) / 2 + cidx;
-        double v = Sacc[e];
-        for (int q = 1; q < acc_copies; ++q) v += Sacc[(size_t)q * acc_n + e];
-        Sp[i] = v;
-      }
+      if (cidx <= r) Sp[i] = Sacc[r * (r + 1) / 2 + cidx];
     }
   }
   SCHUR_MARK(5);
